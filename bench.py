@@ -42,7 +42,7 @@ PARAM_KEYS = ("xyz", "scale", "rot", "sh_0", "sh_rest", "opacity")
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--gaussians", type=int, default=1_000_000)
@@ -64,7 +64,14 @@ def parse():
     ap.add_argument("--allreduce", default="sync", choices=["sync", "overlap"],
                     help="N>1: sync = the step's all-reduce completes before the next step starts (what synchronous training needs; "
                          "headline); overlap = it hides behind the next step's rendering (gradients one step late)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (per-view losses, accumulated gradients at a fixed "
+                         "sample of Gaussians) as DIR/<name>.npy, to compare the outputs of two builds on identical inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.log_scale_range = (0.002, 0.02)
     if a.config == "c4":
         a.gaussians, a.width, a.height = 5_000_000, 3840, 2160
@@ -225,6 +232,27 @@ def load_scene(args):
 def camera_np(i, args):
     from litegs_b200 import scene
     return scene.make_camera(i % args.n_views, args.n_views, args.width, args.height)
+
+
+DUMP_SAMPLE = 65536          # Gaussians whose gradients --dump-outputs writes (59 floats each at sh_degree 3: 15.5 MB)
+
+
+def dump_outputs(out_dir, losses, grads):
+    """--dump-outputs: what a step of render_views hands back to its caller -- the per-view losses it returns and the gradients
+    it accumulated into the dense buffer ("_touched" = the per-chunk marks) -- as float32 DIR/<name>.npy.  The per-Gaussian
+    gradients are written at DUMP_SAMPLE Gaussian slots drawn with a fixed seed (all of them when there are fewer), in
+    ascending slot order, so that every file stays small at any workload size and two runs write the same elements."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"losses": torch.stack([l_.reshape(()) for l_ in losses]), "touched": grads["_touched"]}
+    n = grads["xyz"].shape[-2] * grads["xyz"].shape[-1]
+    idx = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SAMPLE), replace=False))
+    idx_t = torch.from_numpy(idx).to(grads["xyz"].device)
+    for k in PARAM_KEYS:
+        g = grads[k]
+        out[f"grad_{k}"] = g.reshape(*g.shape[:-2], n).index_select(-1, idx_t)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def stage_bytes(stats, S, K):
@@ -501,14 +529,16 @@ def run_ours(args, rank, world, local_rank):
         else:
             a.all_reduce(async_op=False)
 
+    last_losses = []
+
     def step(serial=False, record=False):
         a = accs[step_no["k"] % len(accs)]
         a.wait()                      # overlap mode: this buffer's previous all-reduce (two steps ago) must have landed
         a.zero_()
         if args.level == "B":
-            run_views(lambda j: cams[j], lambda j, img: (img * w).sum(), serial)
+            last_losses[:] = run_views(lambda j: cams[j], lambda j, img: (img * w).sum(), serial)
         else:
-            run_views(lambda j: cams[j], lambda j, img: w, serial)
+            last_losses[:] = run_views(lambda j: cams[j], lambda j, img: w, serial)
         reduce_step(a, record)
         step_no["k"] += 1
 
@@ -539,6 +569,8 @@ def run_ours(args, rank, world, local_rank):
     sampler.mark_end()
     clocks = sampler.stop() if rank == 0 else None
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_losses, accs[(step_no["k"] - 1) % len(accs)].grads())
     comm_ms = sum(a_.elapsed_time(b_) for a_, b_ in comm_events) / max(1, len(comm_events)) if comm_events else 0.0
     # stage attribution / roofline durations: the same steps once more on ONE stream with CUDA events around every
     # C-ABI call (with overlapping streams a kernel's event-to-event time includes the other stream's work).

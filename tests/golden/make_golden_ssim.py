@@ -7,6 +7,10 @@ Inputs are seeded (numpy default_rng(7)): a random image pair and a smooth pair 
 renders where sigma is small), [2,3,37,53]: ragged against every tile size in play (16x16 in the reference, 64x32 ours).
 Stored per mode (0 = SSIM map, 1 = L1 + SSIM loss map with weight 0.2): map, the three partials, and dL/dimg1 for a seeded
 upstream gradient.
+
+Also writes tests/golden/ssim_1080p_sample.npz: the L1 + SSIM loss (weight 0.2) of a seeded 1920x1080 pair, its three partials
+and dL/dimg1 for a seeded upstream gradient (inputs from ``inputs_1080p``), stored at a fixed seeded sample of SAMPLE_1080P
+elements, with each tensor's largest magnitude and the sums of the three inputs (to check that they regenerate).
 """
 import os
 import sys
@@ -35,6 +39,31 @@ def inputs():
     return out, up
 
 
+SAMPLE_1080P = 4096
+
+
+def inputs_1080p(dev):
+    """A 1080p image pair 0.1 apart and an upstream gradient, from torch's CPU generator (seed 2)."""
+    g = torch.Generator(device="cpu").manual_seed(2)
+    x = torch.rand((1, 3, 1080, 1920), generator=g).to(dev)
+    y = (x + 0.1 * (torch.rand((1, 3, 1080, 1920), generator=g).to(dev) - 0.5)).clamp(0, 1)
+    up = torch.randn((1, 3, 1080, 1920), generator=g).to(dev)
+    return x, y, up
+
+
+def sample_1080p(ref, dev):
+    x, y, up = inputs_1080p(dev)
+    idx = np.sort(np.random.default_rng(13).choice(x.numel(), SAMPLE_1080P, replace=False)).astype(np.int64)
+    ti = torch.from_numpy(idx).to(dev)
+    m, d0, d1, d2 = ref.fusedl1ssim_loss(0.2, 0.01 ** 2, 0.03 ** 2, x, y, True)
+    g = ref.fusedl1ssim_loss_backward(0.2, 0.01 ** 2, 0.03 ** 2, x, y, up, d0, d1, d2)
+    store = {"index": idx, "input_sums": np.array([float(t.double().sum()) for t in (x, y, up)])}
+    for k, v in zip(("map", "dm_dmu1", "dm_dsigma1_sq", "dm_dsigma12", "grad"), (m, d0, d1, d2, g)):
+        store[k] = v.reshape(-1)[ti].cpu().numpy()
+        store[f"{k}_absmax"] = np.float64(v.abs().max().item())
+    return store
+
+
 def main():
     outdir = sys.argv[1] if len(sys.argv) > 1 else os.path.join(ROOT, "tests", "golden")
     os.makedirs(outdir, exist_ok=True)
@@ -59,6 +88,9 @@ def main():
             store[f"{name}_l1_{k}"] = v.cpu().numpy()
     path = os.path.join(outdir, "ssim_small.npz")
     np.savez_compressed(path, **store)
+    print("wrote", path, os.path.getsize(path), "bytes")
+    path = os.path.join(outdir, "ssim_1080p_sample.npz")
+    np.savez_compressed(path, **sample_1080p(ref, dev))
     print("wrote", path, os.path.getsize(path), "bytes")
 
 

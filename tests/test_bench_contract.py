@@ -87,3 +87,30 @@ def test_path_bytes_count_only_the_launched_stages():
     assert bench.stage_bytes(st2, 128, 16)["lgs_project_backward"] == 48 * st["Nv"] + (44 + 2 * 236) * st["Nv"]
     src = open(os.path.join(ROOT, "bench.py")).read()
     assert "sum(v for k, v in bytes_per.items())" not in src
+
+
+def test_dump_outputs_writes_the_step_results_at_a_fixed_sample(tmp_path):
+    """--dump-outputs: float32 .npy per returned array, gradients at the same seeded Gaussian sample on every call."""
+    import numpy as np
+    import torch
+    bench = _bench_module()
+    C, S = 600, 128
+    n = C * S
+    g = torch.Generator().manual_seed(0)
+    shapes = {"xyz": (3,), "scale": (3,), "rot": (4,), "sh_0": (1, 3), "sh_rest": (15, 3), "opacity": (1,)}
+    grads = {k: torch.randn((*s, C, S), generator=g) for k, s in shapes.items()}
+    grads["_touched"] = torch.ones(C)
+    losses = [torch.tensor(1.5), torch.tensor(-2.0)]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), losses, grads)
+    names = sorted(f for f in os.listdir(tmp_path / "a"))
+    assert names == sorted(["losses.npy", "touched.npy"] + [f"grad_{k}.npy" for k in shapes])
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in names) <= 64 << 20
+    for f in names:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b), f
+    assert np.array_equal(np.load(tmp_path / "a" / "losses.npy"), [1.5, -2.0])
+    x = np.load(tmp_path / "a" / "grad_sh_rest.npy")
+    assert x.shape == (15, 3, bench.DUMP_SAMPLE)
+    idx = np.sort(np.random.default_rng(0).choice(n, bench.DUMP_SAMPLE, replace=False))
+    assert np.array_equal(x, grads["sh_rest"].reshape(15, 3, n).numpy()[..., idx])

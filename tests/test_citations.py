@@ -1,13 +1,13 @@
 """Every reference citation of the form `<file>:<line>[-<line>]` in the C ABI header, the kernels, the host mirror, the
-oracle and the design documents must resolve against the mounted reference tree: the file exists and has at least that many lines.  Skipped
-where /root/reference is absent (the GPU box)."""
+oracle and the design documents must resolve against the reference tree: the file exists and has at least that many lines.  The
+tree is represented by the line count of each of its source files (tests/golden/reference_tree.json, written by
+tests/golden/make_golden_tree.py)."""
+import json
 import os
 import re
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+TREE = os.path.join(ROOT, "tests", "golden", "reference_tree.json")
 PREFIXES = {"GR/": "litegs/submodules/gaussian_raster/", "fused_ssim/": "litegs/submodules/fused_ssim/", "litegs/": "litegs/"}
 BARE = {"wrapper.py": "litegs/utils/wrapper.py", "optimizer.py": "litegs/training/optimizer.py", "trainer.py": "litegs/training/trainer.py",
         "data.py": "litegs/data.py", "densify.py": "litegs/training/densify.py", "statistic_helper.py": "litegs/utils/statistic_helper.py",
@@ -36,22 +36,18 @@ def _resolve(name):
     return [BARE[name]]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference not mounted")
 def test_reference_citations_resolve():
-    lines_of = {}
+    lines_of = json.load(open(TREE))["line_counts"]
     bad, n = [], 0
     for src in _sources():
         text = open(src, errors="replace").read()
         for m in CITE.finditer(text):
             name, a, b = m.group(1), int(m.group(2)), int(m.group(3) or m.group(2))
-            paths = [os.path.join(REF, c) for c in _resolve(name)]
-            path = next((p for p in paths if os.path.exists(p)), None)
+            path = next((p for p in _resolve(name) if p in lines_of), None)
             n += 1
             if path is None:
                 bad.append((os.path.relpath(src, ROOT), m.group(0), "no such file"))
                 continue
-            if path not in lines_of:
-                lines_of[path] = sum(1 for _ in open(path, errors="replace"))
             if not (1 <= a <= b <= lines_of[path]):
                 bad.append((os.path.relpath(src, ROOT), m.group(0), f"file has {lines_of[path]} lines"))
     assert n > 150, n

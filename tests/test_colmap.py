@@ -1,22 +1,17 @@
 """CPU tests of litegs_b200/colmap.py (SURVEY 8f rank 3: the data format on the input side of the path).
 
 * binary round trip of cameras / images / points3D;
-* the files our writer produces are read by the REFERENCE's own reader (litegs/io_manager/colmap.py, imported from
-  /root/reference with its two heavy imports stubbed) to exactly what was written -- skipped when the tree is absent;
+* the files our writer produces are read by the REFERENCE's own reader (litegs/io_manager/colmap.py) to exactly what was
+  written, through what that reader decoded from them (tests/golden/colmap_reference_reader.npz);
 * camera conversion against the reference's formulas (litegs/data.py:33-51,72-77) and its round trip;
 * initial Gaussians from SfM points against litegs/scene/point.py:7-19 with a brute-force k-NN."""
-import importlib.util
+import hashlib
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 
 from litegs_b200 import colmap, scene
-
-REF = "/root/reference/litegs"
-
 
 def _model(n_pts=300, n_views=4, W=160, H=96, seed=0):
     rng = np.random.default_rng(seed)
@@ -48,59 +43,33 @@ def test_binary_round_trip(tmp_path):
         assert np.array_equal(p2[k].track, p.track)
 
 
-def _reference_reader():
-    """litegs/io_manager/colmap.py imported on its own: `plyfile` (absent here) and `litegs.data` (pulls in cv2/torch
-    datasets) are replaced by stubs that record the constructor arguments."""
-    path = os.path.join(REF, "io_manager", "colmap.py")
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not present")
-    saved = {k: sys.modules.get(k) for k in ("plyfile", "litegs", "litegs.data", "litegs.io_manager", "litegs.io_manager.colmap")}
-    try:
-        ply = types.ModuleType("plyfile"); ply.PlyData = object; ply.PlyElement = object
-        pkg = types.ModuleType("litegs"); pkg.__path__ = [REF]
-        iom = types.ModuleType("litegs.io_manager"); iom.__path__ = [os.path.join(REF, "io_manager")]
-        data = types.ModuleType("litegs.data")
-
-        class PinHoleCameraInfo:
-            def __init__(self, id, width, height, parameters):
-                self.id, self.width, self.height, self.parameters = id, width, height, np.array(parameters)
-
-        class ImageFrame:
-            def __init__(self, id, qvec, tvec, camera_id, name, img_source, xys):
-                self.id, self.qvec, self.tvec, self.camera_id, self.name, self.img_source, self.xys = id, qvec, tvec, camera_id, name, img_source, xys
-
-        data.PinHoleCameraInfo, data.ImageFrame, data.CameraInfo = PinHoleCameraInfo, ImageFrame, object
-        sys.modules.update({"plyfile": ply, "litegs": pkg, "litegs.io_manager": iom, "litegs.data": data})
-        spec = importlib.util.spec_from_file_location("litegs.io_manager.colmap", path)
-        mod = importlib.util.module_from_spec(spec)
-        sys.modules["litegs.io_manager.colmap"] = mod
-        spec.loader.exec_module(mod)
-        return mod
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+READER_MODEL = dict(n_pts=120, n_views=5)
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "colmap_reference_reader.npz")
 
 
 def test_reference_reader_reads_what_we_write(tmp_path):
-    ref = _reference_reader()
-    cams, images, pts = _model(n_pts=120, n_views=5)
-    colmap.write_model(str(tmp_path), cams, images, pts)
-    cam_dict, frames = ref.load_frames(str(tmp_path), "images")
-    assert set(cam_dict) == {1}                                    # only PINHOLE cameras are kept (colmap.py:222-224)
-    assert (cam_dict[1].width, cam_dict[1].height) == (160, 96) and np.array_equal(cam_dict[1].parameters, cams[1].params)
-    assert [f.name for f in frames] == sorted(im.name for im in images.values())
+    """tests/golden/colmap_reference_reader.npz holds what the reference's reader decoded from the files our writer produced
+    for this model, and their SHA-256 (tests/golden/make_golden_tree.py): the files written now are those bytes, and what the
+    reference read from them is exactly what was written."""
+    z = np.load(GOLD)
+    cams, images, pts = _model(**READER_MODEL)
+    d = colmap.write_model(str(tmp_path), cams, images, pts)
+    for f, digest in zip(z["file_names"], z["file_sha256"]):
+        assert hashlib.sha256(open(os.path.join(d, str(f)), "rb").read()).hexdigest() == str(digest), f
+    assert list(z["camera_ids"]) == [1]                            # only PINHOLE cameras are kept (colmap.py:222-224)
+    assert tuple(z["camera_wh"][0]) == (160, 96) and np.array_equal(z["camera_params"][0], cams[1].params)
+    assert list(z["frame_names"]) == sorted(im.name for im in images.values())
     by_name = {im.name: im for im in images.values()}
-    for f in frames:
-        im = by_name[f.name]
-        assert f.id == im.id and np.array_equal(f.qvec, im.qvec) and np.array_equal(f.tvec, im.tvec) and f.camera_id == 1
-        assert np.array_equal(np.asarray(f.xys).reshape(-1, 2), np.asarray(im.xys).reshape(-1, 2))
-    xyz, rgb, err = ref.__dict__["__read_points3D_binary"](os.path.join(str(tmp_path), "sparse", "0", "points3D.bin"))
+    xys = np.split(z["frame_xys"], np.cumsum(z["frame_xys_len"])[:-1])
+    for i, name in enumerate(z["frame_names"]):
+        im = by_name[str(name)]
+        assert z["frame_ids"][i] == im.id and np.array_equal(z["frame_qvec"][i], im.qvec) and np.array_equal(z["frame_tvec"][i], im.tvec)
+        assert z["frame_camera_ids"][i] == 1
+        assert np.array_equal(xys[i], np.asarray(im.xys).reshape(-1, 2))
     want = [pts[k] for k in pts]
-    assert np.array_equal(xyz, np.stack([p.xyz for p in want])) and np.array_equal(rgb, np.stack([p.rgb for p in want]).astype(np.float64))
-    assert np.array_equal(err[:, 0], np.array([p.error for p in want]))
+    assert np.array_equal(z["points_xyz"], np.stack([p.xyz for p in want]))
+    assert np.array_equal(z["points_rgb"], np.stack([p.rgb for p in want]).astype(np.float64))
+    assert np.array_equal(z["points_err"][:, 0], np.array([p.error for p in want]))
 
 
 def test_camera_conversion_matches_reference_formulas():

@@ -1,9 +1,12 @@
 """SURVEY 8f rank 4 -- densification statistics and chunk maintenance -- against their definitions:
  * gpu_driven_pipeline_sparse_op: add / min / max over every dtype the reference dispatches (GR/compact.cu:1221-1336);
- * Morton codes, spatial_refine and chunk AABBs on the device vs the numpy restatement and, when the reference package is
-   staged, vs the reference's own functions (litegs/scene/point.py:22-154, litegs/scene/cluster.py:29-46);
+ * Morton codes, spatial_refine and chunk AABBs on the device vs the numpy restatement and vs what the reference's own
+   functions (litegs/scene/point.py:22-154, litegs/scene/cluster.py:29-46) computed on the same inputs
+   (tests/golden/scene_reference.npz, written by tests/golden/make_golden_scene.py);
  * litegs_b200.statistics.StatisticsHelper fed by Level A and by the fused Level B: same numbers, equal to the ones derived from
    the oracle's raster statistics (statistic_helper.py:82-156,215-243; wrapper.py:501-506)."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -47,18 +50,8 @@ def _morton_numpy(xyz, bits=21):
     return code
 
 
-def _reference_scene_module():
-    from oracle import build_ref
-    import sys
-    path = build_ref.reference_python_path()
-    if path is None:
-        return None
-    from litegs_b200 import shims
-    shims.install()
-    if path not in sys.path:
-        sys.path.insert(1, path)
-    import litegs
-    return litegs.scene
+def _reference_golden():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "scene_reference.npz"))
 
 
 def test_morton_codes_and_spatial_refine(cuda):
@@ -76,22 +69,16 @@ def test_morton_codes_and_spatial_refine(cuda):
     for k in T:
         src = T[k].cpu().numpy().reshape(-1, C * S)
         assert np.array_equal(out[k].cpu().numpy().reshape(-1, C * S), src[:, order_np]), k
-    ref = _reference_scene_module()
-    if ref is not None:
-        # the reference's own spatial_refine in its optimizer form (point.py:104-154: parameters and Adam moments reordered in
-        # place; its tensor form, :94-103, passes a tuple to uncluster and cannot run) and its Morton codes
-        prm = {k: torch.nn.Parameter(T[k].clone()) for k in PARAM_KEYS}
-        opt = torch.optim.Adam([{"params": [prm[k]], "lr": 0.0, "name": k} for k in PARAM_KEYS], lr=0.0, eps=1e-15)
-        for k in PARAM_KEYS:
-            opt.state[prm[k]] = {"step": torch.tensor(0.0), "exp_avg": (T[k] * 0.5).clone(), "exp_avg_sq": (T[k] * T[k]).clone()}
-        r = ref.spatial_refine(True, opt, prm["xyz"])
-        mom, _ = scene.spatial_refine_device({"xyz": T["xyz"], **{f"m_{k}": T[k] * 0.5 for k in PARAM_KEYS}, **{f"v_{k}": T[k] * T[k] for k in PARAM_KEYS}})
-        for k, t in zip(PARAM_KEYS, r):
-            assert torch.equal(t.detach().reshape(out[k].shape), out[k]), k
-            assert torch.equal(opt.state[prm[k]]["exp_avg"].reshape(out[k].shape), mom[f"m_{k}"]), k
-            assert torch.equal(opt.state[prm[k]]["exp_avg_sq"].reshape(out[k].shape), mom[f"v_{k}"]), k
-        import litegs.scene.point as refpoint
-        assert torch.equal(refpoint._gen_morton_code(T["xyz"].reshape(3, -1)), torch.from_numpy(codes).to(cuda))
+    # the reference's own spatial_refine in its optimizer form (point.py:104-154: parameters and Adam moments reordered in place;
+    # its tensor form, :94-103, passes a tuple to uncluster and cannot run) and its Morton codes, bit for bit
+    from tests.golden.make_golden_scene import digest
+    ref = _reference_golden()
+    mom, _ = scene.spatial_refine_device({"xyz": T["xyz"], **{f"m_{k}": T[k] * 0.5 for k in PARAM_KEYS}, **{f"v_{k}": T[k] * T[k] for k in PARAM_KEYS}})
+    for k in PARAM_KEYS:
+        assert digest(out[k]) == str(ref[f"refine_{k}_sha256"]), k
+        assert digest(mom[f"m_{k}"]) == str(ref[f"refine_exp_avg_{k}_sha256"]), k
+        assert digest(mom[f"v_{k}"]) == str(ref[f"refine_exp_avg_sq_{k}_sha256"]), k
+    assert digest(torch.from_numpy(codes)) == str(ref["morton_sha256"])
 
 
 def test_cluster_aabb_device(cuda):
@@ -100,10 +87,8 @@ def test_cluster_aabb_device(cuda):
     o, e = scene.cluster_aabb_device(x, s, q)
     o64, e64 = scene.cluster_aabb(p["xyz"], p["scale"], p["rot"])   # fp64 numpy form of cluster.py:29-46
     assert np.abs(o.cpu().numpy() - o64).max() < 1e-5 and np.abs(e.cpu().numpy() - e64).max() < 1e-5
-    ref = _reference_scene_module()
-    if ref is not None:
-        ro, re_ = ref.cluster.get_cluster_AABB(x, s.exp(), torch.nn.functional.normalize(q, dim=0))
-        assert float((ro - o).abs().max()) < 1e-5 and float((re_ - e).abs().max()) < 1e-5
+    ref = _reference_golden()                                       # the reference's get_cluster_AABB on the same inputs
+    assert np.abs(ref["aabb_origin"] - o.cpu().numpy()).max() < 1e-5 and np.abs(ref["aabb_extend"] - e.cpu().numpy()).max() < 1e-5
     # a box must contain its Gaussians' centres
     assert bool(((x - o[:, :, None]).abs() <= e[:, :, None] + 1e-6).all())
 
